@@ -23,6 +23,9 @@ every rank owns its own 4096 QPs (--batch 1024 gives configs[1]'s literal batch)
             evaluated from the oracle's operation counters on a sample of the
             same workload) / measured solve-kernel time, against the measured
             HBM peak of MEASURED_PEAKS.json.
+
+--dump-outputs DIR writes the results of the last timed device-resident step (rank 0's batch) as DIR/<name>.npy, so
+that two builds can be compared output for output on the same seeded inputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -45,6 +48,7 @@ CPU_SAMPLE = 1024     # QPs per CPU-arm step (a bounded sample of the same workl
 SPARSITY, STRONG_CONVEXITY = 0.15, 1e-2
 EPS_ABS = 1e-9
 KEYS = "HgAbClu"
+DUMP_BYTES = 64 << 20  # cap of --dump-outputs
 
 
 def algorithmic_bytes_per_qp(cnt, n, ne, ni, ncons, batch):
@@ -72,6 +76,22 @@ def compulsory_bytes_per_qp(n, ne, ni):
 def generate(first, count, gen):
     data = [gen("strongly_convex", first + i, N_DIM, N_EQ, N_IN, SPARSITY, STRONG_CONVEXITY) for i in range(count)]
     return {k: np.stack([d[k] for d in data]) for k in KEYS}
+
+
+def dump_outputs(out_dir, res, first):
+    """Write DenseBatch.results() as float64 .npy files: x, y, z, se, si [B, *] and one info_<field> [B] per pqp_info
+    field except the wall-clock *_time ones, plus qp_index [B] (the seed of each row's QP). Above DUMP_BYTES the rows
+    are a fixed sample of the batch (numpy seed 0, sorted), the same for every run with the same --batch."""
+    arrays = {k: res[k] for k in ("x", "y", "z", "se", "si")}
+    arrays.update({"info_" + k: v for k, v in res["info"].items() if not k.endswith("_time")})
+    B = len(res["x"])
+    row_bytes = 8 * (1 + sum(a.size for a in arrays.values()) // B)
+    keep = min(B, DUMP_BYTES // row_bytes)
+    rows = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    arrays["qp_index"] = first + np.arange(B)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(np.asarray(v, dtype=np.float64)[rows]))
 
 
 class ClockSampler:
@@ -310,7 +330,12 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--batch", type=int, default=BATCH_PER_GPU, help="QPs per GPU (default 4096, the north-star batch; BASELINE.json configs[1] literally: 1024)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed device-resident step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -385,6 +410,7 @@ def main():
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
     db.sync()
+    outputs = db.results() if args.dump_outputs and rank == 0 else None  # the last timed step's results
     launches = db.timings()["kernel_launches"] - launches0
     kernel_ms = db.timings()["solve_ms"]  # last solve kernel alone (events around the launch)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
@@ -481,6 +507,8 @@ def main():
                                                       "host_threads": cpu["host_threads"], "cgroup_cpu_quota": cpu_quota()},
         }
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs, rank * B)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

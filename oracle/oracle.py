@@ -7,9 +7,12 @@ may import this module.
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -40,14 +43,15 @@ HESSIAN_ZERO, HESSIAN_DENSE, HESSIAN_DIAGONAL = 0, 1, 2
 
 def use_native() -> str:
     """bench.py only: rebuild the restatement with -march=native ON THE MACHINE THAT RUNS IT (the committed Makefile
-    targets x86-64-v3 so that the prebuilt library of the tests runs on any box) into oracle/_native/ and make this
-    module load that library. Falls back to the portable build if the compiler is missing. Returns the flags used."""
+    targets x86-64-v3 so that the prebuilt library of the tests runs on any box) into a temporary directory, removed at
+    exit (the source tree may be read-only), and make this module load that library. Falls back to the portable build
+    if the compiler is missing. Returns the flags used."""
     global _LIB_PATH, _lib
-    out_dir = os.path.join(_HERE, "_native")
+    out_dir = tempfile.mkdtemp(prefix="pqp_oracle_native_")
+    atexit.register(shutil.rmtree, out_dir, True)
     out = os.path.join(out_dir, "liboracle.so")
     flags = "-O3 -march=native -std=c++17 -fopenmp -fPIC -DNDEBUG"
     try:
-        os.makedirs(out_dir, exist_ok=True)
         subprocess.check_call(["/usr/bin/g++"] + flags.split() + ["-shared", "-o", out, os.path.join(_HERE, "oracle_capi.cpp")],
                               stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         C.CDLL(out)  # must load on this CPU
